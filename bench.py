@@ -207,10 +207,20 @@ def gpu_eager_baseline(dev):
     return res
 
 
+def dump_outputs(path, arrays):
+    """--dump-outputs: what the timed path handed its caller in the last timed step, one float32 DIR/<name>.npy each.
+    The inputs and weights are seeded, so two builds run with the same arguments can be compared output for output."""
+    import numpy as np
+
+    os.makedirs(path, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), t.detach().float().cpu().numpy())
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=30)
+    ap.add_argument("--steps", type=int, default=30, help="number of timed steps")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
@@ -219,7 +229,14 @@ def main():
                     help="bf16x3 (default, the mode of record): split-bf16 GEMMs, fp32 parity; bf16: throughput mode")
     ap.add_argument("--workload", default="pose64",
                     help="pose64 (default) | native | fps | voting | nnd | flow | raster | upnp | refine | ycbv5")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the poses of the last one as DIR/rot.npy [N,3,3] and DIR/trans.npy [N,3] "
+                         "(float32; N = 64 x GPUs, in rank order); pose64 workload, --impl ours")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "pose64"):
+        ap.error("--dump-outputs writes the outputs of the pose64 workload of --impl ours")
     args.warmup = max(args.warmup, 3)
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -337,10 +354,16 @@ def main():
         rots.append(o["rot"].clone() if use_graphs else o["rot"])
         transes.append(o["trans"].clone() if use_graphs else o["trans"])
     if world > 1:
-        all_gather_poses(torch.cat(rots), torch.cat(transes))
+        gathered = all_gather_poses(torch.cat(rots), torch.cat(transes))
     e1.record()
     barrier()
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        if world > 1:   # every rank's poses of every step, in rank order: keep each rank's last step
+            last = [x.view(world, args.steps, BATCH, *x.shape[1:])[:, -1].reshape(world * BATCH, *x.shape[1:]) for x in gathered]
+        else:
+            last = [rots[-1], transes[-1]]
+        dump_outputs(args.dump_outputs, {"rot": last[0], "trans": last[1]})
     launches = L.gdrn_launch_count() - launches0
     if use_graphs:  # graph replays do not pass through the launch counter: count the kernels of one captured forward
         c0_ = L.gdrn_launch_count()

@@ -1,6 +1,6 @@
-"""Pin the oracle: against the reference's own code where it runs here (FPS .cpp compiled into oracle/_ref,
-Python head/PnP/pose classes imported with stubbed third-party deps -> tests/golden/*.npz), and against
-independent formulations elsewhere."""
+"""Pin the oracle: against the reference's own code (FPS .cpp and the vendored-Ceres uncertainty PnP compiled into
+oracle/_ref, Python head/PnP/pose classes imported with stubbed third-party deps; their outputs stored under
+tests/golden/), and against independent formulations elsewhere."""
 import ctypes
 import math
 import os
@@ -15,6 +15,7 @@ from oracle import gdrn_model_oracle as O
 from oracle import ops_oracle as OO
 
 GOLD = os.path.join(ROOT, "tests", "golden")
+GOLD_CPU = os.path.join(GOLD, "ref_cpu_ops.npz")   # tools/make_golden_ref_ops.py cpu
 
 
 def test_fps_oracle_matches_survey_vector():
@@ -30,19 +31,21 @@ def test_fps_oracle_matches_golden_fixture():
         assert (OO.fps(pts, len(idx)) == idx).all(), i
 
 
-def test_fps_oracle_matches_reference_build_when_present():
-    path = os.path.join(ROOT, "oracle", "_ref", "libfps_ref.so")
-    if not os.path.exists(path):
-        pytest.skip("oracle/_ref/libfps_ref.so not built (no /root/reference)")
-    ref = ctypes.CDLL(path)
+def fps_ref_cases():
     rs = np.random.RandomState(5)
     for pn, sn in ((1, 1), (7, 7), (100, 16), (3000, 64), (20000, 128)):
         pts = (rs.rand(pn, 3).astype(np.float32) - 0.5) * 0.3
         if pn == 100:
             pts[10:20] = pts[0]  # duplicates -> zero distances / ties
-        idx = np.zeros(sn, np.int32)
-        ref.farthest_point_sampling_init_center(pts.ctypes.data_as(ctypes.c_void_p), idx.ctypes.data_as(ctypes.c_void_p), pn, sn)
-        assert (OO.fps(pts, sn) == idx).all(), (pn, sn)
+        yield pn, sn, pts
+
+
+def test_fps_oracle_matches_reference_build_when_present():
+    """Against the REFERENCE's own FPS (core/csrc/fps/src/farthest_point_sampling.cpp built into oracle/_ref), whose
+    indices on these clouds are stored in tests/golden/ref_cpu_ops.npz."""
+    g = np.load(GOLD_CPU)
+    for pn, sn, pts in fps_ref_cases():
+        assert (OO.fps(pts, sn) == g["fps/%d_%d" % (pn, sn)]).all(), (pn, sn)
 
 
 def test_head_pnp_pose_oracle_matches_reference_classes():
@@ -282,12 +285,7 @@ def test_baseline_config0_cpu_plumbing():
     pts = rng.uniform(-0.1, 0.1, (8192, 3)).astype(np.float32)
     idx = OO.fps(pts, 64)
     assert len(set(idx.tolist())) == 64 and idx.min() >= 0 and idx.max() < 8192
-    ref_so = os.path.join(ROOT, "oracle", "_ref", "libfps_ref.so")
-    if os.path.exists(ref_so):
-        L = ctypes.CDLL(ref_so)
-        ref = np.zeros(64, np.int32)
-        L.farthest_point_sampling_init_center(pts.ctypes.data_as(ctypes.c_void_p), ref.ctypes.data_as(ctypes.c_void_p), 8192, 64)
-        assert np.array_equal(ref, idx)
+    assert np.array_equal(np.load(GOLD_CPU)["fps/config0"], idx)   # the reference build's indices
 
     tn, vn, hn = 2048, 9, 128
     coords = rng.uniform(0, 64, (tn, 2)).astype(np.float32)
@@ -387,17 +385,23 @@ def upnp_ceres_ref(p2, p3, w, K, init):
     return res
 
 
+UPNP_REF_FIELDS = ("K", "rt", "p2", "p3", "w", "init", "ref")
+
+
+def upnp_ref_problems(prefix):
+    """The stored problems {K, rt, p2, p3, w, init} and the reference's solution ``ref`` of each (ref_cpu_ops.npz)."""
+    g = np.load(GOLD_CPU)
+    return [{f: g["%s/%d/%s" % (prefix, i, f)] for f in UPNP_REF_FIELDS} for i in range(int(g[prefix + "/n"]))]
+
+
 def test_upnp_oracle_pinned_to_vendored_ceres():
     """Pins the uncertainty-PnP oracle (numpy LM) against the REFERENCE's own vendored Ceres 2.0: ceres::Jet autodiff of
     the residual of uncertainty_pnp.cpp:16-34 + ceres::AngleAxisRotatePoint + ceres::TinySolver, built from the headers
-    under /root/reference/core/csrc/uncertainty_pnp/include (oracle/build_ref.py).  Noise-free (the reference main()
-    recipe, :98-156) and noisy problems: same minimiser to 1e-7."""
-    rs = np.random.RandomState(3)
-    if upnp_ceres_ref(*_upnp_problem(rs, 8, 0.0)[2:5], _upnp_problem(rs, 8, 0.0)[0], np.zeros(6) + 0.5) is None:
-        pytest.xfail("oracle/_ref/libupnp_ceres_ref.so not built (python oracle/build_ref.py in the build container)")
-    for trial in range(12):
-        K, rt, p2, p3, w, init = _upnp_problem(rs, 8 + trial, 0.0 if trial % 2 == 0 else 0.5)
-        ref = upnp_ceres_ref(p2, p3, w, K, init)
+    under the reference's core/csrc/uncertainty_pnp/include (oracle/build_ref.py); its solutions are stored in
+    tests/golden/ref_cpu_ops.npz.  Noise-free (the reference main() recipe, :98-156) and noisy problems: same minimiser
+    to 1e-7."""
+    for trial, p in enumerate(upnp_ref_problems("upnp_cpu")):
+        K, rt, p2, p3, w, init, ref = (p[f] for f in UPNP_REF_FIELDS)
         mine = OO.uncertainty_pnp(p2, p3, w, K, init)
         assert np.abs(ref - mine).max() < 1e-7, (trial, ref, mine)
         if trial % 2 == 0:
